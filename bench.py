@@ -8,6 +8,7 @@ query rate()[5m] step 15s over the 2 h (T = 481 windows), gauge schema => RateOv
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            # product arm, one JSON line on rank 0
   python bench.py --impl reference ...                           # reference CPU path (oracle port) on host cores
+  python bench.py ... --dump-outputs DIR                         # also write the last timed step's result arrays as DIR/<name>.npy
 
 A step = one pass of the hot path over the whole resident table (1 kernel launch).  `value` = samples scanned per second
 (Σ numRows of the chunks scanned, the quantity FiloDB counts in samplesScannedCtr) with inputs resident in HBM;
@@ -52,7 +53,52 @@ def parse_args():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the kernel-only sub-records of the other BASELINE configs (C1, C3, C3-const, C4) of the default single-GPU C2 run")
     ap.add_argument("--no-c5", action="store_true", help="skip the C5 sub-record (sum(rate) by(cluster) with the NCCL all-reduce) of the default C2 run")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float64; a fixed, seeded sample of the rows "
+                         "when the result is larger than %d MB), so that two builds can be compared output for output" % (DUMP_LIMIT_BYTES // 1_000_000))
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT_BYTES = 60_000_000
+DUMP_SEED = 20231114
+NPY_HEADER_BYTES = 4096          # generous bound on the header np.save writes in front of the data
+
+
+def dump_row_sample(n_rows, row_bytes):
+    """Rows of an [n_rows x ...] result that fit the dump limit: all of them, or a sorted sample drawn with a fixed seed (the same rows
+    for the same arguments, whichever build runs).  Each sampled row also costs 8 bytes in the `<name>_rows` index array."""
+    fit = (DUMP_LIMIT_BYTES - 2 * NPY_HEADER_BYTES) // (row_bytes + 8)
+    if n_rows <= fit:
+        return None
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n_rows, size=fit, replace=False))
+
+
+def dump_outputs(d, arrays):
+    """Writes each named result array as d/<name>.npy in float64.  `arrays` maps a name to (array, rows), where rows is None (the whole
+    array) or the sorted indices of the first axis the array holds; those go beside it as d/<name>_rows.npy (float64, exact)."""
+    os.makedirs(d, exist_ok=True)
+    total = 0
+    for name, (a, rows) in arrays.items():
+        files = [(name, a)] + ([(name + "_rows", rows)] if rows is not None else [])
+        for fname, x in files:
+            path = os.path.join(d, fname + ".npy")
+            np.save(path, np.ascontiguousarray(x, dtype=np.float64))
+            total += os.path.getsize(path)
+    assert total <= DUMP_LIMIT_BYTES, total
+
+
+def host_rows(a, rows):
+    """The given rows of the first axis of a device tensor or host array (all of them when rows is None), as a host numpy array."""
+    if rows is not None:
+        if hasattr(a, "index_select"):
+            import torch
+            a = a.index_select(0, torch.from_numpy(rows).to(a.device))
+        else:
+            a = a[rows]
+    return a.cpu().numpy() if hasattr(a, "cpu") else np.asarray(a)
 
 
 WORKLOADS = {
@@ -305,11 +351,14 @@ def run_reference(args, rank, world):
             st.add_series(ts, np.cumsum(np.cumsum(obs, axis=1), axis=0), [ROWS_PER_CHUNK, ROWS - ROWS_PER_CHUNK])
         start, step, end, window = T0_MS, STEP, T0_MS + 7200000, WINDOW
         def one_h():
-            st.query(o.FN_RATE, start, step, end, window, aggr=True, group_ids=np.zeros(K, np.int32), n_groups=1, q=0.99)
+            return st.query(o.FN_RATE, start, step, end, window, aggr=True, group_ids=np.zeros(K, np.int32), n_groups=1, q=0.99)
         for _ in range(args.warmup): one_h()
         t0 = time.perf_counter()
-        for _ in range(args.steps): one_h()
+        for _ in range(args.steps): res = one_h()
         dt = (time.perf_counter() - t0) / args.steps
+        if args.dump_outputs:
+            hv, hempty, hq = res
+            dump_outputs(args.dump_outputs, {"values": (hv, None), "empty": (hempty, None), "quantile": (hq, None)})
         val = K * ROWS / dt
         print(json.dumps({"impl": "reference", "metric": "samples/s scanned+aggregated (rate over 10M series); % HBM roofline", "value": val, "unit": "samples/s",
                           "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt * 1e3, "higher_is_better": True, "scaling": "weak",
@@ -331,14 +380,17 @@ def run_reference(args, rank, world):
     groups = o.synth_group_ids(42, 0, S, n_groups) if n_groups else None
 
     def one():
-        st.query(getattr(o, fn_name), start, step, end, window, cumulative=cumulative, aggr=getattr(o, aggr_name),
-                 group_ids=groups, n_groups=max(n_groups, 1), threads=cores, reuse_out=True)
+        return st.query(getattr(o, fn_name), start, step, end, window, cumulative=cumulative, aggr=getattr(o, aggr_name),
+                        group_ids=groups, n_groups=max(n_groups, 1), threads=cores, reuse_out=True)
     for _ in range(args.warmup):
         one()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        one()
+        res = one()
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:      # [series x T] for the sample of S series, or [groups x T]
+        rows = dump_row_sample(res.shape[0], res.shape[1] * 8)
+        dump_outputs(args.dump_outputs, {"values": (host_rows(res, rows), rows)})
     samples = S * ROWS
     val = samples / dt
     line = {"impl": "reference", "metric": "samples/s scanned+aggregated (rate over 10M series); % HBM roofline", "value": val, "unit": "samples/s",
@@ -487,8 +539,10 @@ def run_c4(args, rank, world, local_rank):
     start, step, end, window = T0_MS, STEP, T0_MS + 7200000, WINDOW
     T = capi.num_windows(start, step, end)
 
+    last = {}
+
     def one():
-        ctx.query_hist(tab, capi.FN_RATE, start, step, end, window, aggr=capi.AGG_SUM, quantile=0.99, want_values=False)
+        last["quantile"] = ctx.query_hist(tab, capi.FN_RATE, start, step, end, window, aggr=capi.AGG_SUM, quantile=0.99, want_values=False)
         return ctx.last_stats
     st0 = one()
     assert st0["samples_scanned"] == ti.n_samples, (st0, ti.n_samples)
@@ -500,6 +554,8 @@ def run_c4(args, rank, world, local_rank):
     torch.cuda.synchronize()
     if dist: dist.barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"quantile": (last["quantile"], None)})      # [groups x T], histogram_quantile(0.99, ...)
     ms = float(np.sum(kns)) / 1e6 / args.steps
     if dist:
         t = torch.tensor([ms], device="cuda"); dist.all_reduce(t, op=dist.ReduceOp.MAX); ms = float(t.item())
@@ -648,6 +704,11 @@ def main():
     torch.cuda.synchronize()
     if dist: dist.barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        # what a caller of the step receives: the [series x T] rates of this rank's series, or the presented [groups x T] aggregate
+        res = out.view(S, T) if aggr == capi.AGG_NONE else (final if world > 1 else out).view(n_groups, T)
+        rows = dump_row_sample(res.shape[0], T * 8)
+        dump_outputs(args.dump_outputs, {"values": (host_rows(res, rows), rows)})
     ms = e0.elapsed_time(e1) / args.steps
     ms_per_rank = [ms]
     if dist:

@@ -27,3 +27,24 @@ def test_numpy_generator_models_agree():
         assert (bench.gen_hist_series_np(seed, gid, rows, nb, reset) == sr.gen_hist_series(seed, gid, rows, nb, reset)).all()
     g = bench.synth_group_ids(42, 1000, 64, 7)
     assert list(g) == [sr.group_id(42, 1000 + i, 7) for i in range(64)]
+
+
+def test_bench_dump_outputs_are_fixed_and_bounded(tmp_path, oracle):
+    # bench.py --dump-outputs: a result too large for the limit is sampled by rows, the same rows every time; the files are float64 and two
+    # runs with the same arguments write the same bits
+    import subprocess
+    import sys
+    import bench
+    row_bytes = 481 * 8
+    rows = bench.dump_row_sample(10_000_000, row_bytes)
+    assert (rows == bench.dump_row_sample(10_000_000, row_bytes)).all() and (np.diff(rows) > 0).all() and rows[-1] < 10_000_000
+    assert rows.size * (row_bytes + 8) + 2 * bench.NPY_HEADER_BYTES <= bench.DUMP_LIMIT_BYTES
+    assert bench.dump_row_sample(1000, row_bytes) is None
+    got = []
+    for run in ("a", "b"):
+        subprocess.run([sys.executable, bench.__file__, "--impl", "reference", "--workload", "c2", "--series", "300", "--cpu-series", "300",
+                        "--steps", "2", "--warmup", "0", "--dump-outputs", str(tmp_path / run)], check=True, capture_output=True)
+        assert sorted(p.name for p in (tmp_path / run).iterdir()) == ["values.npy"]
+        got.append(np.load(tmp_path / run / "values.npy"))
+    assert got[0].dtype == np.float64 and got[0].shape == (300, 481) and np.isfinite(got[0]).any()
+    assert (got[0].view(np.uint64) == got[1].view(np.uint64)).all()
